@@ -17,6 +17,10 @@ all-reduce for o and down), strong scaling.
 --impl reference times the reference's own CPU path for this hot path (TorchAtenLinear's int4pack fused op,
 restated in oracle/gptq_oracle.py::CpuFusedLinear) on the host cores; each step is a bounded sample
 (1 of the 32 decoder layers).
+
+--dump-outputs DIR writes, after the timed steps, the last hidden state of the last decode step (decode.npy) and of the
+last prefill pass (prefill.npy) as float32.  Weights and inputs are seeded, so runs with the same arguments compute the
+same thing and two builds can be compared output for output.
 """
 import argparse
 import json
@@ -25,8 +29,10 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -59,6 +65,32 @@ def load_traffic():
 def algorithmic_bytes(K, N, gs, bits, M):
     G = K // gs
     return K * N * bits // 8 + G * N * 2 + G * (N * bits // 32) * 4 + M * K * 2 + M * N * 2
+
+
+def make_input(M, hidden, seed, device):
+    """Activations of one pass [M, hidden] fp16, seeded like the weights (synth_layer): the same in every run.
+    Drawn on the device in fp32 and then cast, like the unseeded inputs before: a decode input copied in from the host
+    instead measured 0.4% slower decode (B200, 1000 W power limit)."""
+    gen = torch.Generator(device=device).manual_seed(seed)
+    return (torch.randn(M, hidden, device=device, generator=gen) * 0.5).to(torch.float16)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each [rows, cols] host array as <out_dir>/<name>.npy in float32.  When they would exceed DUMP_BYTES in all,
+    every array keeps every k-th row only, with the smallest k that fits: k follows from the shapes alone, so the sample
+    is the same in every run."""
+    def nbytes(k):
+        return sum(4 * -(-a.shape[0] // k) * a.shape[1] for a in arrays.values())
+
+    k = 1
+    while nbytes(k) > DUMP_BYTES:
+        k += 1
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a[::k].float().numpy())
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -545,7 +577,13 @@ def main():
                     help="EXPERIMENTAL: decode tier v2 (b2q_decode2.cu; sets B2Q_DECODE_V2=1), result marked experimental")
     ap.add_argument("--fused-allreduce", action="store_true",
                     help="EXPERIMENTAL (N > 1): row-parallel matmul + all-reduce in one launch (b2q_decode_allreduce)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last decode step's and prefill pass's outputs to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     global OVERLAP_CHUNKS
     OVERLAP_CHUNKS = args.overlap_chunks
     if args.decode_v2:
@@ -605,7 +643,7 @@ def main():
     weights_total = sum(CFG[kk] * CFG[nn_] for _, kk, nn_, _ in LINEARS) * args.layers
 
     # ---------------- decode: kernel-resident timing (inputs already in HBM) ----------------
-    x_static = (torch.randn(1, hidden, device=device) * 0.5).to(torch.float16)
+    x_static = make_input(1, hidden, seed=1, device=device)
     g_dec, out_dec = capture(stack, x_static, world)
     for _ in range(args.warmup):
         g_dec.replay()
@@ -619,7 +657,7 @@ def main():
     finite = bool(torch.isfinite(out_dec).all())
 
     # ---------------- decode e2e: host buffers, H2D + graph + D2H every step ----------------
-    x_host = (torch.randn(1, hidden) * 0.5).to(torch.float16).pin_memory()
+    x_host = x_static.cpu().pin_memory()
     y_host = torch.empty(1, hidden, dtype=torch.float16).pin_memory()
     if world > 1:
         dist.barrier()
@@ -640,7 +678,7 @@ def main():
     phase("decode timed")
     # ---------------- prefill: M tokens through the same 224 layers ----------------
     Mp = args.prefill_tokens
-    xp = (torch.randn(Mp, hidden, device=device) * 0.5).to(torch.float16)
+    xp = make_input(Mp, hidden, seed=2, device=device)
     g_pre, out_pre = capture(stack, xp, world)
     it_pre = args.prefill_iters or max(3, min(args.steps, 10))
     for _ in range(3):
@@ -664,6 +702,10 @@ def main():
     pre_e2e_ms = (time.perf_counter() - t0) / it_pre * 1e3
 
     phase("prefill timed")
+    if args.dump_outputs and rank == 0:
+        # the host copies of the last decode step and prefill pass: what a caller of the timed path receives
+        dump_outputs(args.dump_outputs, {"decode": y_host, "prefill": yp_host})
+        phase(f"outputs written to {args.dump_outputs}")
     # ---------------- the other BASELINE configs + batched decode + competitor kernels ----------------
     extra, competitors = {}, None
     if not args.no_extra and args.layers == CFG["layers"]:

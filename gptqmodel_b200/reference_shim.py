@@ -17,8 +17,8 @@ in their own `__dict__` (gptqmodel/utils/importer.py:110-127), ranks them by the
   * `post_init()` / `forward()` / `dequantize_weight()` / `list_buffers()` come from the mixin; `post_init()` ends in the
     base's `post_init()` (adapter initialisation, qlinear/__init__.py:224-234).
 The file a maintainer adds is shown in INTEGRATION.md §2; tests/test_reference_shim.py builds the class against a
-stand-in hierarchy with the reference's exact constructor signatures and, when /root/reference is present, against the
-unmodified reference classes themselves.
+stand-in hierarchy with the reference's exact constructor signatures and compares it with what the same class did on the
+unmodified reference classes (recorded in tests/golden/shim_reference.json).
 """
 from __future__ import annotations
 

@@ -1,9 +1,13 @@
 #!/usr/bin/env python
-"""Authoring-container check (needs /root/reference): build gptqmodel_b200.reference_shim's class on the UNMODIFIED
-reference base `GPTQQuantLinear`, construct it the way `create_quant_module` does (gptqmodel/utils/model.py:630-647), and
-run the reference's own discovery walk over it.  Prints one JSON line; tests/test_reference_shim.py runs it in a
-subprocess so the stubbed third-party modules never leak into the test process.
+"""Record tests/golden/shim_reference.json from the UNMODIFIED reference (needs its source tree, imported as in
+make_golden.py): build gptqmodel_b200.reference_shim's class on the reference base `GPTQQuantLinear`, construct it the
+way `create_quant_module` does (gptqmodel/utils/model.py:630-647), and run the reference's own discovery walk over it.
+Also records the reference's constructor / validate() signatures and the SUPPORTS_* attributes its base classes leave
+to the kernel, which tests/test_reference_shim.py's stand-in hierarchy must restate.
+
+    python tests/golden/check_shim.py
 """
+import inspect
 import json
 import os
 import sys
@@ -19,7 +23,7 @@ make_golden.import_reference()
 import torch  # noqa: E402
 from gptqmodel.adapter.adapter import Lora  # noqa: E402
 from gptqmodel.models._const import DEVICE, PLATFORM  # noqa: E402
-from gptqmodel.nn_modules.qlinear import BaseQuantLinear, GPTQQuantLinear  # noqa: E402
+from gptqmodel.nn_modules.qlinear import BaseQuantLinear, GPTQQuantLinear, GroupedQuantLinear  # noqa: E402
 from gptqmodel.quantization import FORMAT, METHOD  # noqa: E402
 from gptqmodel.utils.backend import BACKEND  # noqa: E402
 
@@ -91,4 +95,22 @@ m5 = B200Linear(bits=5, group_size=64, desc_act=False, sym=False, in_features=25
                 format=FORMAT.GPTQ_P)
 out["bits3"] = dict(qweight=list(m3.qweight.shape), qzeros=list(m3.qzeros.shape), kbits=m3.kbits, planar=bool(m3.planar))
 out["bits5"] = dict(qweight=list(m5.qweight.shape), qzeros=list(m5.qzeros.shape), kbits=m5.kbits, planar=bool(m5.planar))
-print("SHIM_JSON " + json.dumps(out))
+
+
+def signature(fn):
+    return [[p.name, p.kind.name, None if p.default is inspect.Parameter.empty else repr(p.default)]
+            for p in inspect.signature(fn).parameters.values()]
+
+
+interface = {
+    "signatures": {"BaseQuantLinear.__init__": signature(BaseQuantLinear.__init__),
+                   "GPTQQuantLinear.__init__": signature(GPTQQuantLinear.__init__),
+                   "BaseQuantLinear.validate": signature(BaseQuantLinear.validate)},
+    "required_supports": {c.__name__: sorted(n for n, v in vars(c).items() if n.startswith("SUPPORTS") and v is None)
+                          for c in (BaseQuantLinear, GroupedQuantLinear)},
+}
+with open(os.path.join(HERE, "shim_reference.json"), "w") as f:
+    json.dump({"source": "ModelCloud/GPTQModel gptqmodel/nn_modules/qlinear/__init__.py, recorded by "
+                         "tests/golden/check_shim.py", "interface": interface, "shim": out}, f, indent=1, sort_keys=True)
+    f.write("\n")
+print("wrote shim_reference.json")
